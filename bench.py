@@ -26,11 +26,15 @@ A "step" is one pass of the hot path over one batch of synthetic tasks:
 * ``payload4k``: ``synthetic 4 KB-payload map, 1e6 tasks`` (configs[3], per GPU): the HBM-bound kernels at
                  8.2 GB per launch (dispatch_payload_map_tma, gather_bulk).
 
-``cpu_baseline`` / ``--impl reference`` time the UNMODIFIED reference pool (``baseline/_ref/fiber``: a
-git-ignored copy of /root/reference/fiber made by ``__graft_entry__.build()`` with the one constant
-``socket_lib = "nanomsg" -> "zmq"`` flipped because nnpy is not installable offline) on this box's host
-cores; if that copy is missing or fails, the oracle port of ZPool (``oracle/zpool_port.py``) stands in
-and the line says ``kind: "port"``.
+``cpu_baseline`` / ``--impl reference`` time the UNMODIFIED reference pool on this box's host cores: its
+``fiber`` package compiled to bytecode in ``oracle/_ref/fiber`` by ``__graft_entry__.build()``
+(``oracle/ref_pyc.py``, git-ignored, with the one constant ``socket_lib = "nanomsg" -> "zmq"`` because nnpy
+is not installable offline); if that build is missing or fails, the oracle port of ZPool
+(``oracle/zpool_port.py``) stands in and the line says ``kind: "port"``.
+
+``--steps K`` is the number of timed steps of every GPU leg (the CPU baseline arms keep fixed repetitions).  ``--dump-outputs DIR`` writes what the headline
+leg's last timed step computed (see ``dump_pi_outputs``) as ``DIR/<name>.npy``; the inputs depend only on the
+arguments, so two builds can be compared output for output.
 """
 import argparse
 import ctypes
@@ -49,7 +53,7 @@ sys.path.insert(0, ROOT)
 PI_TASKS = 10 ** 8
 PAYLOAD_TASKS = 10 ** 6
 CPU_SAMPLE_TASKS = 10 ** 6
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 
 
 def load_peaks():
@@ -284,6 +288,14 @@ class Dist:
     def all_true(self, flag):
         return self.sum_i64(0 if flag else 1) == 0
 
+    def gather_objects(self, obj):
+        """Every rank's picklable `obj`, in rank order, on every rank."""
+        if self.world == 1:
+            return [obj]
+        out = [None] * self.world
+        self.dist.all_gather_object(out, obj)
+        return out
+
     def finish(self):
         if self.world > 1:
             if self.comm is not None:
@@ -431,8 +443,36 @@ def oracle_pi_equal(got_u8, first):
     return all(_parallel(jobs))
 
 
+DUMP_SAMPLE = 1 << 20
+DUMP_BLOCK = 10 ** 4
+
+
+def dump_pi_outputs(out_dir, got_u8, first, total_count, dist):
+    """Write what a caller of the headline map receives -- the ordered is_inside results of every rank's
+    tasks [first, first + n) and the job's count -- as float64/float32 .npy files on rank 0 (about 12 MB
+    in all; every rank calls this, its part travels to rank 0):
+      pi_inside_index.npy  float64  a fixed sample of task indices (seed 0, sorted, unique; DUMP_SAMPLE / world
+                                    draws per rank, ranks in order)
+      pi_inside_sample.npy float32  the results at those indices (0 or 1)
+      pi_block_counts.npy  float64  the number of true results in every block of DUMP_BLOCK consecutive tasks
+      pi_count.npy         float64  [the count over all ranks]"""
+    import numpy as np
+    n = got_u8.shape[0]
+    idx = np.unique(np.random.default_rng(0).integers(0, n, DUMP_SAMPLE // dist.world))
+    blocks = np.add.reduceat(got_u8, np.arange(0, n, DUMP_BLOCK), dtype=np.int64)
+    parts = dist.gather_objects((first, got_u8[idx], blocks))
+    if dist.rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("pi_inside_index", np.concatenate([f + idx for f, _, _ in parts]).astype(np.float64)),
+                      ("pi_inside_sample", np.concatenate([s for _, s, _ in parts]).astype(np.float32)),
+                      ("pi_block_counts", np.concatenate([b for _, _, b in parts]).astype(np.float64)),
+                      ("pi_count", np.array([total_count], dtype=np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 # ------------------------------------------------------------------------------------------------
-# CPU arm: the reference's own pool (baseline/_ref/fiber), or its oracle port, in a child process
+# CPU arm: the reference's own pool (oracle/_ref/fiber), or its oracle port, in a child process
 # ------------------------------------------------------------------------------------------------
 def _cpu_child(spec):
     """Runs in a fresh interpreter (`bench.py --cpu-child <json>`): the reference pool's workers re-import
@@ -479,7 +519,9 @@ def _cpu_child(spec):
 
 
 def cpu_arm(work, P, n=CPU_SAMPLE_TASKS, reps=3, warm=1, timeout=420):
-    """-> (result dict, kind).  Tries the real reference first, then the port."""
+    """-> (result dict, kind).  Tries the real reference first, then the port; a port result that stands in
+    for a failed reference arm says why in its ``impl``."""
+    import tempfile
     kinds = ["reference", "port"] if os.path.isdir(os.path.join(REF_DIR, "fiber")) else ["port"]
     last_err = None
     for kind in kinds:
@@ -489,11 +531,18 @@ def cpu_arm(work, P, n=CPU_SAMPLE_TASKS, reps=3, warm=1, timeout=420):
         env.pop("RANK", None)
         spec = {"kind": kind, "P": P, "n": n, "reps": reps, "warm": warm, "work": work}
         try:
-            cp = subprocess.run([sys.executable, os.path.abspath(__file__), "--cpu-child", json.dumps(spec)], env=env, cwd=ROOT,
-                                stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=timeout)
+            # the reference logs to /tmp/fiber.log.<process> by default: a private directory keeps files another user
+            # left there from failing the arm, and leaves nothing behind
+            with tempfile.TemporaryDirectory(prefix="fbr_cpu_arm_") as logs:
+                env["FIBER_LOG_FILE"] = os.path.join(logs, "fiber.log")
+                cp = subprocess.run([sys.executable, os.path.abspath(__file__), "--cpu-child", json.dumps(spec)], env=env, cwd=ROOT,
+                                    stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=timeout)
             for ln in cp.stdout.splitlines():
                 if ln.startswith("CPU_CHILD_RESULT "):
-                    return json.loads(ln[len("CPU_CHILD_RESULT "):]), kind
+                    res = json.loads(ln[len("CPU_CHILD_RESULT "):])
+                    if last_err:
+                        res["impl"] = "%s (standing in: %s)" % (res.get("impl"), last_err[-200:])
+                    return res, kind
             last_err = "%s arm printed no result (rc %d): %s" % (kind, cp.returncode, cp.stderr[-300:])
         except subprocess.TimeoutExpired:
             last_err = "%s arm timed out after %d s" % (kind, timeout)
@@ -622,7 +671,7 @@ def inprocess_pool_e2e(n_gpus, steps):
         step.last = res
     for _ in range(3):
         step()
-    k = max(3, min(steps, 10))
+    k = steps
     t0 = time.perf_counter()
     for _ in range(k):
         step()
@@ -752,9 +801,9 @@ def run_multi_gpu(args, dist, dev):
         store.wait(["fbr_fused_done"])
     dist.barrier()
     from fiber_b200 import comm as C
-    t_ok, t_algbw, t_busbw, t_ms = allreduce_bench(64 * 1024 * 1024, steps=max(5, args.steps), warmup=3, device=cuda)
+    t_ok, t_algbw, t_busbw, t_ms = allreduce_bench(64 * 1024 * 1024, steps=args.steps, warmup=3, device=cuda)
     if comm is not None:
-        ar_ok, algbw, busbw, ar_ms = C.allreduce_bench(comm, 64 * 1024 * 1024, steps=max(5, args.steps), warmup=3)
+        ar_ok, algbw, busbw, ar_ms = C.allreduce_bench(comm, 64 * 1024 * 1024, steps=args.steps, warmup=3)
     else:
         ar_ok, algbw, busbw, ar_ms = t_ok, t_algbw, t_busbw, t_ms
     return {
@@ -781,7 +830,7 @@ def run_multi_gpu(args, dist, dev):
 # ------------------------------------------------------------------------------------------------
 # parzen (BASELINE.json configs[2])
 # ------------------------------------------------------------------------------------------------
-def run_parzen(dev, traffic, with_cpu):
+def run_parzen(dev, traffic, with_cpu, steps):
     """102 window widths over the 10 000 x 2 sample set of examples/parzen_estimation.py:32-40 through
     apply_async (as the example) and starmap(chunksize=1); fp32 body = the north-star's path."""
     import numpy as np
@@ -802,18 +851,18 @@ def run_parzen(dev, traffic, with_cpu):
 
     out = {"workload": "parzen_estimation: %d samples x %d dims (seed 123), %d widths, fp32 window test (BASELINE.json configs[2])"
                        % (n, xs.shape[1], len(widths))}
-    for name, fn, reps in (("apply_async_x102", job_apply, 5), ("starmap_chunksize1", job_star, 20)):
+    for name, fn in (("apply_async_x102", job_apply), ("starmap_chunksize1", job_star)):
         for _ in range(2):
             res = fn()
         pool.reset_stats()
         t0 = time.perf_counter()
-        for _ in range(reps):
+        for _ in range(steps):
             res = fn()
-        dt = (time.perf_counter() - t0) / reps
+        dt = (time.perf_counter() - t0) / steps
         st = pool.stats()
-        out[name] = {"ms_per_job": 1e3 * dt, "tasks_per_s": len(widths) / dt, "kernel_launches_per_job": st["dispatch_launches"] / reps,
-                     "kernel_us_per_job": 1e3 * st["dispatch_ms"] / reps, "h2d_bytes_per_job": st["h2d_bytes"] // reps,
-                     "d2h_bytes_per_job": st["d2h_bytes"] // reps}
+        out[name] = {"ms_per_job": 1e3 * dt, "tasks_per_s": len(widths) / dt, "kernel_launches_per_job": st["dispatch_launches"] / steps,
+                     "kernel_us_per_job": 1e3 * st["dispatch_ms"] / steps, "h2d_bytes_per_job": st["h2d_bytes"] // steps,
+                     "d2h_bytes_per_job": st["d2h_bytes"] // steps}
     star = np.asarray(res)
     # parity: k_n vs the CPU fp32 restatement (exact) and vs fp64 (boundary samples only), density rtol 1e-6
     mism, ok = 0, True
@@ -925,8 +974,11 @@ def run_ours(args, dist):
     launches_value = st["dispatch_launches"] + st["gather_launches"]
     dispatch_ms = st["dispatch_ms"] / max(1, st["dispatch_launches"])
     # FULL parity of the device-resident ordered output of the last timed step (outside the timed loop)
-    value_parity = oracle_pi_equal(eng.d2h(out_dev, PI_TASKS), my_first)
-    value_parity = dist.all_true(value_parity)
+    value_out = eng.d2h(out_dev, PI_TASKS)
+    value_parity = dist.all_true(oracle_pi_equal(value_out, my_first))
+    if args.dump_outputs:
+        dump_pi_outputs(args.dump_outputs, value_out, my_first, total_count, dist)
+    del value_out
 
     # ---- the gather leg: same map, task records shuffled inside each wave -> records + ring + gather_ordered
     leg["flags"] = _abi.FBR_SHUFFLE
@@ -1015,7 +1067,7 @@ def run_ours(args, dist):
         pl_drain()
         eng.release_deferred()
         eng.stats(reset=True)
-        k_ring = max(3, args.steps // 2)
+        k_ring = args.steps
         t_plr = timed_steps(dist, k_ring, 0, pl_step, pl_drain, clocks.windows)
         eng.release_deferred()
         spr = eng.stats()
@@ -1141,7 +1193,7 @@ def run_ours(args, dist):
         for _ in range(2):
             pl_e2e_step()
         pool.reset_stats()
-        k_pl = max(3, min(args.steps, 5))
+        k_pl = args.steps
         t_pl_e2e = timed_steps(dist, k_pl, 0, pl_e2e_step, None, clocks.windows)
         sp2 = pool.stats()
         got = np.asarray(pl_e2e_step.last)
@@ -1221,7 +1273,7 @@ def run_ours(args, dist):
     # ---------------- parzen (config 3) and the CPU baseline (rank 0, N=1) -------------------------------------
     parzen = cpu = None
     if rank == 0 and not args.skip_parzen:
-        parzen = run_parzen(dev, traffic, with_cpu=(world == 1 and not args.skip_cpu))
+        parzen = run_parzen(dev, traffic, with_cpu=(world == 1 and not args.skip_cpu), steps=args.steps)
     if rank == 0 and world == 1 and not args.skip_cpu:
         cores = os.cpu_count() or 1
         try:
@@ -1271,14 +1323,19 @@ def run_ours(args, dist):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of every GPU leg (the CPU baseline arms keep their own fixed repetitions)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--skip-payload", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-parzen", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline map's last timed step (sampled results, block counts, count) as DIR/<name>.npy")
     ap.add_argument("--cpu-child", default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.cpu_child:
         _cpu_child(json.loads(args.cpu_child))
         return 0
