@@ -128,29 +128,22 @@ static int occ_thread(int index_mode) {
 static void launch_payload_map(const void* wpv, int grid, void* sv) {
     const WaveParams& wp = *(const WaveParams*)wpv;
     cudaStream_t s = (cudaStream_t)sv;
-    // contiguous records: TMA-staged, warp-specialised kernel (2 CTAs of 5 warps per SM); strided
-    // records (arg_stride > 4096) keep the register-streaming kernel
-    static const bool use_tma = !(getenv("FBR_DISPATCH_TMA") && atoi(getenv("FBR_DISPATCH_TMA")) == 0);
-    if (use_tma && wp.arg_stride == kPayloadBytes) {
+    // contiguous records: TMA-staged, warp-specialised kernel (2 CTAs of 5 warps per SM; a 6+3-stage variant at 1 CTA/SM
+    // was no faster, DESIGN.md section 6); strided records (arg_stride > 4096) keep the register-streaming kernel
+    if (wp.arg_stride == kPayloadBytes) {
         int sm = 148, dev = 0;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, dev);
-        static const bool deep = getenv("FBR_TMA_DEEP") && atoi(getenv("FBR_TMA_DEEP")) != 0;
-        int per_sm = deep ? 1 : 2;
-        if (const char* e = getenv("FBR_DISPATCH_OCC")) per_sm = std::max(1, std::min(per_sm, atoi(e)));
-        const int g = (int)std::min<uint32_t>(wp.n_units, (uint32_t)(sm * per_sm));
-        if (deep) dispatch_payload_map_tma_kernel<6, 3><<<g, 160, tma_map::smem_bytes(6, 3), s>>>(wp);
-        else dispatch_payload_map_tma_kernel<3, 2><<<g, 160, tma_map::kSmemBytes, s>>>(wp);
+        const int g = (int)std::min<uint32_t>(wp.n_units, (uint32_t)(sm * 2));
+        dispatch_payload_map_tma_kernel<3, 2><<<g, 160, tma_map::kSmemBytes, s>>>(wp);
         return;
     }
     dispatch_payload_map_kernel<<<grid, kThreads, 0, s>>>(wp);
 }
 static int occ_payload_map(int) {
     cudaFuncSetAttribute(dispatch_payload_map_tma_kernel<3, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tma_map::kSmemBytes);
-    cudaFuncSetAttribute(dispatch_payload_map_tma_kernel<6, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tma_map::smem_bytes(6, 3));
     cudaFuncAttributes at;
     cudaFuncGetAttributes(&at, (const void*)dispatch_payload_map_tma_kernel<3, 2>);   // force-load
-    cudaFuncGetAttributes(&at, (const void*)dispatch_payload_map_tma_kernel<6, 3>);
     return occ_of((const void*)dispatch_payload_map_kernel);
 }
 static void launch_payload_checksum(const void* wpv, int grid, void* sv) {
@@ -251,7 +244,6 @@ struct Worker {
     int numa_node = -1;                    // host NUMA node the GPU hangs off (-1 unknown)
     int sm_count = 0;
     cudaStream_t s_in = nullptr, s_comp = nullptr, s_out = nullptr;
-    cudaStream_t s_out2 = nullptr;         // FBR_TWO_OUT_STREAMS=1: copy-outs alternate between s_out and s_out2 (by staging half)
     cudaStream_t s_gath = nullptr;         // higher-priority stream for gathers that overlap the next dispatch
     bool prev_wave_overlap = false;        // the previous wave used only its half of the ring
     cudaStream_t s_push = nullptr;         // a stream of the ROOT worker's device: its copy engine pushes this worker's argument waves
@@ -288,7 +280,7 @@ static int worker_occ(Worker& w, int func_id, const BodyEntry& body, bool index_
 
 struct TimedPair { cudaEvent_t a, b; };
 
-struct PartCtx {                          // constants of one worker's block of one map
+struct PartPlan {                         // how one worker's block of one map runs (plan_part)
     uint32_t unit = 0, slot_stride = 0, R = 0, sum_kind = 0;
     bool args_dev = false, out_dev = false, full_window = false, host_args = false, resilient = false, keep_on_device = false;
     bool overlap = false;                 // gather(w) on s_gath concurrently with dispatch(w+1); ring used in halves
@@ -300,11 +292,14 @@ struct PartCtx {                          // constants of one worker's block of 
                                           // records into this worker's staging halves over NVLink (host_args machinery)
     bool direct = false;                  // contiguous, unshuffled, non-resilient block: the dispatch kernel stores every
                                           // unit at its final index (no ring, no task records, no gather launch)
+    uint64_t wave_tasks_cap = 0;          // tasks per wave: every wave but the last has exactly this many
+    uint64_t args_limit_bytes = 0;        // host arguments end here (n_items records); 0 = n_tasks * arg_stride
+};
+
+struct PartCtx : PartPlan {               // ... and the memory submit_part acquired for it
     const uint8_t* d_shared = nullptr;
     uint8_t* window_base = nullptr;       // device output of a FULL_WINDOW part
     const uint8_t* args_full = nullptr;   // device-resident arguments of the whole map (args_dev / resilient)
-    uint64_t wave_tasks_cap = 0;
-    uint64_t args_limit_bytes = 0;        // host arguments end here (n_items records); 0 = n_tasks * arg_stride
 };
 
 struct SeqPart {
@@ -403,6 +398,9 @@ void SubmitThread_loop_impl(SubmitThread* t) {
 }
 
 static uint64_t round_up(uint64_t x, uint64_t m) { return (x + m - 1) / m * m; }
+
+// ring arena size of a pool created with `ring_bytes` (0: the default, 256 MiB)
+static uint64_t pool_ring_bytes(uint64_t ring_bytes) { return round_up(ring_bytes ? ring_bytes : (256ull << 20), 4096); }
 
 static uint64_t pin_class(uint64_t bytes) {
     uint64_t c = 4096;
@@ -528,7 +526,6 @@ static int worker_init(fbr_pool* p, Worker& w, int device) {
     CK(cudaStreamCreateWithFlags(&w.s_in, cudaStreamNonBlocking));
     CK(cudaStreamCreateWithFlags(&w.s_comp, cudaStreamNonBlocking));
     CK(cudaStreamCreateWithFlags(&w.s_out, cudaStreamNonBlocking));
-    CK(cudaStreamCreateWithFlags(&w.s_out2, cudaStreamNonBlocking));
     {
         int lo_prio = 0, hi_prio = 0;
         CK(cudaDeviceGetStreamPriorityRange(&lo_prio, &hi_prio));
@@ -581,7 +578,6 @@ static void worker_destroy(Worker& w) {
     if (w.s_in) cudaStreamSynchronize(w.s_in);
     if (w.s_comp) cudaStreamSynchronize(w.s_comp);
     if (w.s_out) cudaStreamSynchronize(w.s_out);
-    if (w.s_out2) { cudaStreamSynchronize(w.s_out2); cudaStreamDestroy(w.s_out2); }
     if (w.s_gath) { cudaStreamSynchronize(w.s_gath); cudaStreamDestroy(w.s_gath); }
     if (w.s_push) {                        // lives on the root worker's device
         cudaSetDevice(w.push_root_device);
@@ -618,11 +614,11 @@ static void worker_destroy(Worker& w) {
 
 // Claim-unit size: near the body's preferred size, a multiple of the API chunksize when the chunk
 // is smaller (so chunk boundaries coincide with unit boundaries), and a multiple of 16/R tasks so
-// every full slot is 16 B aligned on both sides of the gather.
+// every full slot is 16 B aligned on both sides of the gather.  `chunksize` 0 stands for the default, 32.
 static uint32_t pick_unit(const BodyEntry& b, uint32_t chunksize, uint64_t n_tasks, int sm_count, uint64_t ring_bytes) {
     uint32_t pref = b.unit_tasks;
     if (pref == 1) return 1;
-    if (const char* e = getenv("FBR_UNIT_TASKS")) pref = (uint32_t)std::max(16, atoi(e));   // tuning knob (profiles/pi_perf.py)
+    if (chunksize == 0) chunksize = 32;
     // a unit's results (and its argument records) must fit the ring arenas
     const uint64_t per_task = std::max<uint64_t>(std::max(b.result_bytes, b.arg_bytes), 1);
     while (pref > 1 && (uint64_t)pref * per_task > ring_bytes / 2) pref >>= 1;
@@ -638,6 +634,136 @@ static uint32_t pick_unit(const BodyEntry& b, uint32_t chunksize, uint64_t n_tas
     unit = (uint32_t)round_up(unit, align);
     while (unit > align && (uint64_t)unit * per_task > ring_bytes) unit -= align;   // chunk-aligned unit too big for the ring
     return unit;
+}
+
+// Tasks [*b0, *b1) of block `i` when `count` tasks are cut into `nw` contiguous blocks on the boundaries of the
+// map-level claim unit (block partition == PUSH round-robin with chunk = block, SURVEY.md 8(e)); empty if *b1 <= *b0.
+static void block_range(const BodyEntry& body, uint32_t chunksize, uint64_t count, int nw, int i, int sm_count,
+                        uint64_t ring_bytes, uint64_t* b0, uint64_t* b1) {
+    const uint32_t unit = pick_unit(body, chunksize, (count + nw - 1) / nw, sm_count, ring_bytes);
+    const uint64_t units_per = ((count + unit - 1) / unit + nw - 1) / nw;
+    *b0 = std::min<uint64_t>(count, (uint64_t)i * units_per * unit);
+    *b1 = std::min<uint64_t>(count, (uint64_t)(i + 1) * units_per * unit);
+}
+
+// How worker `worker`'s block [first, first + count) of map `d` runs: its claim unit, its data path and the size of
+// its waves.  Host arithmetic only -- no CUDA call, and the pool's state comes in through the arguments -- so the
+// schedule can be checked without a device (fbr_internal_plan_part).  `root_alive`: worker 0, which holds
+// device-resident arguments and output, is alive; `has_out`: the map has a result buffer (the caller's `out` or the
+// engine's pinned segment; maps with FBR_RESULTS_ON_DEVICE have none).
+static int plan_part(const BodyEntry& body, const fbr_map_desc_t& d, uint64_t first, uint64_t count, int worker,
+                     bool root_alive, int sm_count, uint64_t ring_bytes, uint32_t pool_flags, bool has_out, PartPlan* out) {
+    PartPlan c;
+    c.R = body.result_bytes;
+    c.resilient = (d.flags & FBR_RESILIENT) != 0;
+    c.args_dev = (d.flags & FBR_ARGS_DEVICE) != 0;
+    c.out_dev = (d.flags & FBR_OUT_DEVICE) != 0;
+    c.keep_on_device = (d.flags & FBR_RESULTS_ON_DEVICE) != 0;
+    // Output resident on worker 0, computed by another worker: kernels storing over NVLink top out near 510 GB/s
+    // (TMA bulk or register stores alike), a copy engine pushes at the peer-copy rate (~770 GB/s).  So the block is
+    // computed into the local out-staging halves and each wave is pushed to the root by this worker's copy engine,
+    // overlapping the next wave's kernel (DESIGN.md section 6).
+    c.peer_out = c.out_dev && worker != 0 && !c.resilient && !(d.flags & FBR_FULL_WINDOW);
+    // Bit-packed bool results are small (1/8 B per task): instead of staging them in HBM and copying them out wave
+    // by wave (6 x (2 MB D2H + ~8 us set-up) = the critical path of the e2e step), the dispatch kernel stores them
+    // straight into the pinned host segment (zero copy): the PCIe writes spread over the whole kernel.
+    // Measured (C ABI, 1e8 index tasks, 12.5 MB of results): 0.304 ms per map against 0.349 ms staged + copied in 6 waves.
+    c.zero_copy = body.result_kind == FBR_RES_BITS8 && !c.out_dev && !c.resilient && !c.keep_on_device &&
+                  !(d.flags & (FBR_FULL_WINDOW | FBR_SHUFFLE | FBR_VIA_RING | FBR_NO_ZERO_COPY)) && has_out;
+    c.full_window = (c.out_dev && !c.peer_out) || c.resilient || c.keep_on_device || (d.flags & FBR_FULL_WINDOW) || c.zero_copy;
+    // Device-resident arguments on worker 0, consumed by another worker: worker 0's copy engine pushes them wave by
+    // wave into this worker's staging halves, the same wave / staging machinery as host-resident arguments.
+    c.peer_push = c.args_dev && d.arg_stride != 0 && worker != 0 && !c.resilient && root_alive;
+    c.host_args = d.arg_stride != 0 && !c.resilient && (!c.args_dev || c.peer_push);
+    c.unit = pick_unit(body, d.chunksize, count, sm_count, ring_bytes);
+    c.slot_stride = (uint32_t)round_up((uint64_t)c.unit * c.R, 16);
+    const uint32_t unit = c.unit, R = c.R;
+    if (d.n_items && d.arg_stride && body.result_kind == FBR_RES_BITS8)
+        c.args_limit_bytes = d.n_items * (uint64_t)(d.arg_stride / 8);   // a byte-task's record is 8 items
+    if (d.flags & FBR_WANT_SUM) {
+        if (!(body.flags & FBR_BODY_SUMMABLE)) return fail(FBR_EINVAL, "body %s results cannot be summed", body.name.c_str());
+        c.sum_kind = 1;   // the dispatch kernel folds sum(results) while they are in registers
+    }
+
+    // Opt-in (FBR_POOL_OVERLAP): gather(w) runs on a second, higher-priority stream while the next
+    // wave's / next map's dispatch kernel computes; the ring is then used in alternating halves.
+    // Measured on the pi map (ALU-bound dispatch + HBM-bound gather, maps pipelined back to back):
+    // 0.3837 vs 0.3876 ms/step -- the gather is only 9 % of the step and the two kernels contend for
+    // SM slots, so it is off by default.
+    c.overlap = c.full_window && !c.resilient && (pool_flags & FBR_POOL_OVERLAP) != 0;
+    // Direct placement: a contiguous, unshuffled, non-resilient block needs neither task records nor the
+    // ring -- unit t of a wave is tasks [wave_first + t*unit, ...) and its results belong at exactly that
+    // index of the ordered window, so the dispatch kernel stores them there and no gather is launched.
+    // (Shuffled arrival, several attempts per unit and FBR_VIA_RING keep the ring + gather_ordered path.)
+    const bool unit_ok = ((uint64_t)unit * R) % 16 == 0 || unit == 1;   // full vectors are stored 16 B at a time
+    const bool base_ok = !c.out_dev || (((uintptr_t)d.out + first * R) & 15) == 0;
+    c.direct = !c.resilient && !(d.flags & (FBR_SHUFFLE | FBR_VIA_RING)) && unit_ok && base_ok;
+
+    // wave capacity in claim units
+    uint64_t units_cap = c.direct ? (1ull << 31) :   // 32-bit unit counter; a direct wave needs no ring space
+        std::min<uint64_t>(kRecCapacity, (c.overlap ? ring_bytes / 2 : ring_bytes) / c.slot_stride);
+    if (c.host_args) units_cap = std::min<uint64_t>(units_cap, ring_bytes / ((uint64_t)unit * d.arg_stride));
+    if (!c.full_window) units_cap = std::min<uint64_t>(units_cap, ring_bytes / ((uint64_t)unit * R));
+    if (units_cap == 0) return fail(FBR_ENOMEM, "ring_bytes=%llu too small for one claim unit of %u tasks", (unsigned long long)ring_bytes, unit);
+    c.wave_tasks_cap = units_cap * unit;
+    // Host-resident output: cut large maps into ~8 waves (>= 8 MiB of results each) so the D2H of
+    // wave w overlaps the kernels of wave w+1 instead of trailing one monolithic launch.  The waves are equal: ramps,
+    // tapers and pyramids of wave sizes were measured and lost (profiles/r02_peer_sweep.txt, DESIGN.md section 6).
+    if (!c.full_window || c.host_args) {
+        const uint64_t bytes_per_task = std::max<uint64_t>(R, c.host_args ? d.arg_stride : 0);
+        // a wave must carry enough kernel time to hide its launches: 8 MiB of byte results is ~22 us of
+        // pi dispatch; a byte of bit-packed results stands for 8 tasks, so 1 MiB is the same work
+        const uint64_t min_wave_bytes = body.result_kind == FBR_RES_BITS8 ? (1ull << 20) : (8ull << 20);
+        const uint64_t min_wave_tasks = round_up(std::max<uint64_t>(1, min_wave_bytes / bytes_per_task), unit);
+        // 8 waves for ~100 MB maps, up to 64 for multi-GB ones (~64 MiB per wave): the first wave's
+        // H2D and the last wave's D2H are the only copies nothing overlaps with
+        uint64_t n_waves = std::min<uint64_t>(64, std::max<uint64_t>(8, count * bytes_per_task / (64ull << 20)));
+        // small outputs (bit-packed bools): per-copy set-up weighs more: T_kernel/n + n * 8 us is flattest at n = 5..6
+        if (body.result_kind == FBR_RES_BITS8 && !c.host_args) n_waves = 6;
+        const uint64_t share = round_up((count + n_waves - 1) / n_waves, unit);
+        c.wave_tasks_cap = std::min(c.wave_tasks_cap, std::max(min_wave_tasks, share));
+    }
+    *out = c;
+    return FBR_OK;
+}
+
+// Which gather kernel (see kernels.cuh) places a wave of `n_units` ring slots into its ordered window, and its grid.
+// `out_aligned`: the window starts on a 16-byte boundary.  Host arithmetic only, like plan_part.
+enum GatherKind { GATHER_FLAT, GATHER_ROWS, GATHER_BULK };
+struct GatherPlan {
+    GatherKind kind;
+    int grid;
+    uint32_t group_slots;                 // slots per ticket (rows / bulk)
+    bool reverse;                         // rows: newest slot first
+};
+static GatherPlan plan_gather(const PartPlan& cx, bool out_aligned, uint32_t n_units, int sm_count, int occ_gather,
+                              int occ_gather_rows) {
+    const bool rows_ok = out_aligned && (uint64_t)cx.unit * cx.R == cx.slot_stride && cx.slot_stride % 4096 == 0;
+    // TMA bulk pipeline for slots of whole 16 KB chunks (4 KB slots: the rows kernel is faster, 37 vs 41 us on the pi wave)
+    if (rows_ok && !cx.resilient && cx.slot_stride % bulk::kChunk == 0) {
+        // ONE warp per SM saturates HBM (measured 104 % of the copy peak vs 102.5 % with two);
+        // ~256 KB of ring per ticket (<= 32 slots: one header per lane), >= ~8 tickets per CTA
+        const uint64_t max_ctas = (uint64_t)sm_count;
+        const uint32_t group_slots = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(
+            std::min<uint64_t>(bulk::kGroup, (256u << 10) / cx.slot_stride), n_units / (8 * max_ctas)));
+        const uint32_t n_groups = (n_units + group_slots - 1) / group_slots;
+        return {GATHER_BULK, (int)std::min<uint64_t>(n_groups, max_ctas), group_slots, false};
+    }
+    if (rows_ok) {
+        // ~128 KB of ring per ticket, but never fewer than ~4 tickets per resident CTA (small waves);
+        // big slots (>= 32 KB): 4 fat streams per SM measured best (100 % of the copy peak vs 99 %)
+        const int occ_g = cx.slot_stride >= (32u << 10) ? std::min(occ_gather_rows, 4) : occ_gather_rows;
+        const uint64_t max_ctas = (uint64_t)sm_count * occ_g;
+        const uint32_t group_slots = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((128u << 10) / cx.slot_stride, n_units / (4 * max_ctas)));
+        const uint32_t n_groups = (n_units + group_slots - 1) / group_slots;
+        // waves that fit the L2 are gathered newest-slot-first (see the kernel)
+        const bool reverse = (uint64_t)n_units * cx.slot_stride <= (128ull << 20);
+        return {GATHER_ROWS, (int)std::min<uint64_t>(n_groups, max_ctas), group_slots, reverse};
+    }
+    const uint64_t total_vec = (uint64_t)n_units * (cx.slot_stride >> 4);
+    const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((total_vec + kThreads * 4 - 1) / (kThreads * 4),
+                                                                   (uint64_t)sm_count * occ_gather));
+    return {GATHER_FLAT, grid, 0, false};
 }
 
 static void shuffle_records(TaskRecord* r, uint32_t n, uint64_t seed) {
@@ -769,7 +895,6 @@ static int run_wave(fbr_pool* p, SeqState& st, SeqPart& part, const BodyEntry& b
     int occ_d = worker_occ(w, st.func_id, body, d.arg_stride == 0);
     if (body.max_ctas_per_sm) occ_d = std::min(occ_d, body.max_ctas_per_sm);
     if (ov && occ_d > 1) occ_d -= 1;     // leave SM slots for the concurrently running gather CTAs
-    if (const char* e = getenv("FBR_DISPATCH_OCC")) occ_d = std::max(1, std::min(occ_d, atoi(e)));
     const int grid_d = (int)std::min<uint64_t>(n_units, (uint64_t)w.sm_count * occ_d);
     TimedPair td{nullptr, nullptr}, tg{nullptr, nullptr};
     if (timing) {
@@ -811,49 +936,16 @@ static int run_wave(fbr_pool* p, SeqState& st, SeqPart& part, const BodyEntry& b
         gp.lost_count = cx.resilient ? &w.d_ctrl[slot].lost_count : nullptr;
         gp.lost_units = part.d_lost;
         gp.lost_capacity = part.lost_cap;
-        const uint64_t total_vec = (uint64_t)n_units * (cx.slot_stride >> 4);
-        const int grid_g = (int)std::max<uint64_t>(1, std::min<uint64_t>((total_vec + kThreads * 4 - 1) / (kThreads * 4),
-                                                                          (uint64_t)w.sm_count * w.occ_gather));
-        // kernel choice for this wave (see kernels.cuh): TMA bulk pipeline, row streaming, or flat
-        const bool aligned = (((uintptr_t)gp.out & 15) == 0) && (((uint64_t)cx.unit * cx.R) == cx.slot_stride);
-        const bool rows_ok = aligned && (cx.slot_stride % 4096 == 0) && getenv("FBR_GATHER_FLAT") == nullptr;
-        const bool bulk_ok = rows_ok && !cx.resilient &&
-                             (cx.slot_stride % bulk::kChunk == 0 || getenv("FBR_BULK_SMALL") != nullptr) &&   // 4 KB slots: rows kernel is faster (37 vs 41 us on the pi wave)
-                             (cx.slot_stride <= bulk::kChunk || cx.slot_stride % bulk::kChunk == 0) &&
-                             !(getenv("FBR_GATHER_BULK") && atoi(getenv("FBR_GATHER_BULK")) == 0);
+        const GatherPlan g = plan_gather(cx, ((uintptr_t)gp.out & 15) == 0, n_units, w.sm_count, w.occ_gather, w.occ_gather_rows);
         uint32_t* gticket = w.d_tickets + kTickets + (wno % kTickets);   // zero at launch, re-armed below
-        if (bulk_ok) {
-            const uint32_t stage = std::min<uint32_t>(cx.slot_stride, bulk::kChunk);
-            const size_t smem_bytes = (size_t)bulk::kStages * stage;
-            // big chunks: ONE warp per SM saturates HBM (measured 104 % of the copy peak vs 102.5 % with two);
-            // 4 KB chunks need more CTAs to keep enough bytes in flight
-            int per_sm = stage >= bulk::kChunk ? 1 : (int)std::min<size_t>(8, (200u << 10) / smem_bytes);
-            if (const char* e = getenv("FBR_GATHER_OCC")) per_sm = std::max(1, atoi(e));
-            // ~256 KB of ring per ticket (<= 32 slots: one header per lane), >= ~8 tickets per CTA
-            const uint64_t max_ctas = (uint64_t)w.sm_count * per_sm;
-            uint32_t group_slots = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(
-                std::min<uint64_t>(bulk::kGroup, (256u << 10) / cx.slot_stride), n_units / (8 * max_ctas)));
-            if (const char* e = getenv("FBR_BULK_GROUP")) group_slots = std::max(1, std::min(32, atoi(e)));
-            const uint32_t n_groups = (n_units + group_slots - 1) / group_slots;
-            const int grid_b = (int)std::min<uint64_t>(n_groups, max_ctas);
-            gather_bulk_kernel<<<grid_b, 32, smem_bytes, s_g>>>(gp, gticket, stage, group_slots);
+        if (g.kind == GATHER_BULK) {
+            gather_bulk_kernel<<<g.grid, 32, (size_t)bulk::kStages * bulk::kChunk, s_g>>>(gp, gticket, bulk::kChunk, g.group_slots);
             CK(cudaMemsetAsync(gticket, 0, sizeof(uint32_t), s_g));
-        } else if (rows_ok) {
-            // ~128 KB of ring per ticket, but never fewer than ~4 tickets per resident CTA (small waves);
-            // big slots (>= 32 KB): 4 fat streams per SM measured best (100 % of the copy peak vs 99 %)
-            int occ_g = cx.slot_stride >= (32u << 10) ? std::min(w.occ_gather_rows, 4) : w.occ_gather_rows;
-            if (const char* e = getenv("FBR_GATHER_OCC")) occ_g = std::max(1, std::min(occ_g, atoi(e)));
-            const uint64_t max_ctas = (uint64_t)w.sm_count * occ_g;
-            const uint32_t group_slots = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((128u << 10) / cx.slot_stride, n_units / (4 * max_ctas)));
-            const uint32_t n_groups = (n_units + group_slots - 1) / group_slots;
-            const int grid_r = (int)std::min<uint64_t>(n_groups, max_ctas);
-            // waves that fit the L2 are gathered newest-slot-first (see the kernel); FBR_GATHER_REVERSE=0/1 overrides
-            bool reverse = (uint64_t)n_units * cx.slot_stride <= (128ull << 20);
-            if (const char* e = getenv("FBR_GATHER_REVERSE")) reverse = atoi(e) != 0;
-            gather_rows_kernel<<<grid_r, kThreads, 0, s_g>>>(gp, gticket, group_slots, reverse);
+        } else if (g.kind == GATHER_ROWS) {
+            gather_rows_kernel<<<g.grid, kThreads, 0, s_g>>>(gp, gticket, g.group_slots, g.reverse);
             CK(cudaMemsetAsync(gticket, 0, sizeof(uint32_t), s_g));
         } else {
-            gather_ordered_kernel<<<grid_g, kThreads, 0, s_g>>>(gp);
+            gather_ordered_kernel<<<g.grid, kThreads, 0, s_g>>>(gp);
         }
         CK(cudaGetLastError());
         if (timing) {
@@ -870,10 +962,9 @@ static int run_wave(fbr_pool* p, SeqState& st, SeqPart& part, const BodyEntry& b
         cudaEvent_t wd;
         CK(cudaEventCreateWithFlags(&wd, cudaEventDisableTiming));
         if (!cx.full_window) {
-            // one copy-out stream by default; alternating two (FBR_TWO_OUT_STREAMS=1) was measured and did not pay:
-            // 0.362 vs 0.347 ms per 1e8-task map over PCIe, 3.40 vs 3.41 ms for the NVLink push of 2 GB
-            static const bool two_out = getenv("FBR_TWO_OUT_STREAMS") && atoi(getenv("FBR_TWO_OUT_STREAMS")) != 0;
-            cudaStream_t so = (half && two_out) ? w.s_out2 : w.s_out;
+            // one copy-out stream: alternating two did not pay (0.362 vs 0.347 ms per 1e8-task map over PCIe, 3.40 vs
+            // 3.41 ms for the NVLink push of 2 GB)
+            cudaStream_t so = w.s_out;
             CK(cudaStreamWaitEvent(so, w.ev_comp[rw], 0));
             if (cx.peer_out) {      // this worker's copy engine writes the wave into the root's ordered output (posted NVLink writes)
                 CK(cudaMemcpyPeerAsync((uint8_t*)st.out + wave_first * cx.R, p->workers[0].device, w.d_out[half], w.device, wt * cx.R, so));
@@ -899,19 +990,10 @@ static int finish_round(fbr_pool* p, SeqState& st, SeqPart& part, bool copy_wind
     const PartCtx& cx = part.cx;
     const int slot = part.ctrl_slot;
     const int last_rw = (int)((w.wave_no - 1) % kRecWindows);
-    // A block whose results never pass through the copy-out stream (device-resident output, zero-copy stores into the
-    // pinned segment) finishes on the compute stream itself: its control block follows its last kernel without a
-    // cross-stream hop.  Everything else finishes on s_out, behind its copy-outs.
-    // (Off: a copy on the compute stream puts a DMA hop between back-to-back kernels of pipelined maps, which costs
-    // them what a blocking map() gains.  FBR_FINISH_ON_COMP=1 enables it for A/B runs.)
-    static const bool finish_on_comp = getenv("FBR_FINISH_ON_COMP") && atoi(getenv("FBR_FINISH_ON_COMP")) != 0;
-    const bool on_comp = finish_on_comp && cx.direct && cx.full_window && !cx.resilient && (cx.zero_copy || cx.out_dev || cx.keep_on_device);
-    cudaStream_t sf = on_comp ? w.s_comp : w.s_out;
-    if (!on_comp) {
-        CK(cudaStreamWaitEvent(w.s_out, w.ev_comp[last_rw], 0));
-        CK(cudaStreamWaitEvent(w.s_out, w.ev_out[0], 0));      // copy-outs issued on either out stream are complete
-        CK(cudaStreamWaitEvent(w.s_out, w.ev_out[1], 0));
-    }
+    // The round finishes on s_out, behind the block's last kernels and its copy-outs, even when nothing was copied out:
+    // a copy on the compute stream would put a DMA hop between the back-to-back kernels of pipelined maps.
+    cudaStream_t sf = w.s_out;
+    CK(cudaStreamWaitEvent(sf, w.ev_comp[last_rw], 0));
     if (copy_window && cx.full_window && !cx.out_dev && !cx.keep_on_device && !cx.zero_copy && part.count) {
         CK(cudaMemcpyAsync((uint8_t*)st.out + part.first * cx.R, cx.window_base, part.count * cx.R, cudaMemcpyDeviceToHost, sf));
         STAT_ADD(p, d2h_bytes, part.count * cx.R);
@@ -931,53 +1013,22 @@ static int submit_part(fbr_pool* p, SeqState& st, SeqPart& part, const BodyEntry
     const fbr_map_desc_t& d = st.desc;
     PartCtx& cx = part.cx;
     CK(cudaSetDevice(w.device));
-    cx.R = body.result_bytes;
-    cx.resilient = (d.flags & FBR_RESILIENT) != 0;
-    cx.args_dev = (d.flags & FBR_ARGS_DEVICE) != 0;
-    cx.out_dev = (d.flags & FBR_OUT_DEVICE) != 0;
-    cx.keep_on_device = (d.flags & FBR_RESULTS_ON_DEVICE) != 0;
-    {
-        // Output resident on worker 0, computed by another worker: kernels storing over NVLink top out near 510 GB/s
-        // (TMA bulk or register stores alike), a copy engine pushes at the peer-copy rate (~770 GB/s).  So the block is
-        // computed into the local out-staging halves and each wave is pushed to the root by this worker's copy engine,
-        // overlapping the next wave's kernel (FBR_PEER_OUT=0: the kernel stores into the root's memory itself).
-        static const bool out_off = getenv("FBR_PEER_OUT") && atoi(getenv("FBR_PEER_OUT")) == 0;
-        cx.peer_out = cx.out_dev && part.worker != 0 && !cx.resilient && !out_off && !(d.flags & FBR_FULL_WINDOW);
-    }
-    {
-        // Bit-packed bool results are small (1/8 B per task): instead of staging them in HBM and copying them out wave
-        // by wave (6 x (2 MB D2H + ~8 us set-up) = the critical path of the e2e step), the dispatch kernel can store them
-        // straight into the pinned host segment (zero copy): the PCIe writes spread over the whole kernel.
-        // Measured (C ABI, 1e8 index tasks, 12.5 MB of results): 0.304 ms per map against 0.349 ms staged + copied in 6 waves.
-        static const int zc = getenv("FBR_ZERO_COPY") ? atoi(getenv("FBR_ZERO_COPY")) : 1;
-        cx.zero_copy = zc != 0 && body.result_kind == FBR_RES_BITS8 && !cx.out_dev && !cx.resilient && !cx.keep_on_device &&
-                       !(d.flags & (FBR_FULL_WINDOW | FBR_SHUFFLE | FBR_VIA_RING | FBR_NO_ZERO_COPY)) && st.out != nullptr;
-    }
-    cx.full_window = (cx.out_dev && !cx.peer_out) || cx.resilient || cx.keep_on_device || (d.flags & FBR_FULL_WINDOW) || cx.zero_copy;
-    cx.host_args = d.arg_stride != 0 && !cx.args_dev && !cx.resilient;
-    {
-        // device-resident arguments on worker 0, consumed by another worker: stream them through the staging halves,
-        // pushed wave by wave by the root's copy engine (FBR_PEER_PUSH=0: the kernel loads them over NVLink itself)
-        static const bool push_off = getenv("FBR_PEER_PUSH") && atoi(getenv("FBR_PEER_PUSH")) == 0;
-        if (cx.args_dev && d.arg_stride != 0 && part.worker != 0 && !cx.resilient && !push_off && !p->workers[0].dead) {
-            if (w.s_push == nullptr) {
-                const int root = p->workers[0].device;
-                CK(cudaSetDevice(root));
-                cudaError_t e = cudaStreamCreateWithFlags(&w.s_push, cudaStreamNonBlocking);
-                if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&w.s_push2, cudaStreamNonBlocking);
-                for (int i = 0; i < kRecWindows && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&w.ev_push[i], cudaEventDisableTiming);
-                cudaSetDevice(w.device);
-                if (e != cudaSuccess) return fail(FBR_ECUDA, "creating the push stream on device %d failed: %s", root, cudaGetErrorString(e));
-                w.push_root_device = root;
-            }
-            cx.peer_push = true;
-            cx.host_args = true;       // same wave / staging machinery as host-resident arguments
-        }
-    }
-    const uint32_t cs = d.chunksize ? d.chunksize : 32u;
-    cx.unit = pick_unit(body, cs, part.count, w.sm_count, p->ring_bytes);
-    cx.slot_stride = (uint32_t)round_up((uint64_t)cx.unit * cx.R, 16);
+    const int prc = plan_part(body, d, part.first, part.count, part.worker, !p->workers[0].dead, w.sm_count, p->ring_bytes,
+                              p->flags, st.out != nullptr, &cx);
+    if (prc != FBR_OK) return prc;
     const uint32_t unit = cx.unit, R = cx.R;
+
+    // push streams: a stream of the root device whose copy engine pushes this worker's argument waves
+    if (cx.peer_push && w.s_push == nullptr) {
+        const int root = p->workers[0].device;
+        CK(cudaSetDevice(root));
+        cudaError_t e = cudaStreamCreateWithFlags(&w.s_push, cudaStreamNonBlocking);
+        if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&w.s_push2, cudaStreamNonBlocking);
+        for (int i = 0; i < kRecWindows && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&w.ev_push[i], cudaEventDisableTiming);
+        cudaSetDevice(w.device);
+        if (e != cudaSuccess) return fail(FBR_ECUDA, "creating the push stream on device %d failed: %s", root, cudaGetErrorString(e));
+        w.push_root_device = root;
+    }
 
     // control block
     if (w.ctrl_free.empty()) return fail(FBR_ENOMEM, "more than %d maps in flight on worker %d", kCtrlSlots, part.worker);
@@ -1002,8 +1053,6 @@ static int submit_part(fbr_pool* p, SeqState& st, SeqPart& part, const BodyEntry
         }
     }
 
-    if (d.n_items && d.arg_stride && body.result_kind == FBR_RES_BITS8)
-        cx.args_limit_bytes = d.n_items * (uint64_t)(d.arg_stride / 8);   // a byte-task's record is 8 items
     // arguments that stay device-resident for the whole map
     if (cx.args_dev && !cx.peer_push) {
         cx.args_full = (const uint8_t*)d.args;
@@ -1020,50 +1069,6 @@ static int submit_part(fbr_pool* p, SeqState& st, SeqPart& part, const BodyEntry
                                (const uint8_t*)d.args + part.first * (uint64_t)d.arg_stride, abytes, cudaMemcpyHostToDevice, w.s_in));
         STAT_ADD(p, h2d_bytes, abytes);
         cx.args_full = (const uint8_t*)part.d_args_full;
-    }
-
-    // Opt-in (FBR_POOL_OVERLAP): gather(w) runs on a second, higher-priority stream while the next
-    // wave's / next map's dispatch kernel computes; the ring is then used in alternating halves.
-    // Measured on the pi map (ALU-bound dispatch + HBM-bound gather, maps pipelined back to back):
-    // 0.3837 vs 0.3876 ms/step -- the gather is only 9 % of the step and the two kernels contend for
-    // SM slots, so it is off by default.
-    cx.overlap = cx.full_window && !cx.resilient && (p->flags & FBR_POOL_OVERLAP) != 0;
-    // Direct placement: a contiguous, unshuffled, non-resilient block needs neither task records nor the
-    // ring -- unit t of a wave is tasks [wave_first + t*unit, ...) and its results belong at exactly that
-    // index of the ordered window, so the dispatch kernel stores them there and no gather is launched.
-    // (Shuffled arrival, several attempts per unit and FBR_VIA_RING keep the ring + gather_ordered path.)
-    {
-        static const bool env_off = getenv("FBR_DIRECT") && atoi(getenv("FBR_DIRECT")) == 0;
-        const bool unit_ok = ((uint64_t)unit * R) % 16 == 0 || unit == 1;   // full vectors are stored 16 B at a time
-        const bool base_ok = !cx.out_dev || (((uintptr_t)d.out + part.first * R) & 15) == 0;
-        cx.direct = !env_off && !cx.resilient && !(d.flags & (FBR_SHUFFLE | FBR_VIA_RING)) && unit_ok && base_ok;
-    }
-    // wave capacity in claim units
-    uint64_t units_cap = cx.direct ? (1ull << 31) :   // 32-bit unit counter; a direct wave needs no ring space
-        std::min<uint64_t>(kRecCapacity, (cx.overlap ? p->ring_bytes / 2 : p->ring_bytes) / cx.slot_stride);
-    if (cx.host_args) units_cap = std::min<uint64_t>(units_cap, p->ring_bytes / ((uint64_t)unit * d.arg_stride));
-    if (!cx.full_window) units_cap = std::min<uint64_t>(units_cap, p->ring_bytes / ((uint64_t)unit * R));
-    if (units_cap == 0) return fail(FBR_ENOMEM, "ring_bytes=%llu too small for one claim unit of %u tasks", (unsigned long long)p->ring_bytes, unit);
-    cx.wave_tasks_cap = units_cap * unit;
-    // Host-resident output: cut large maps into ~8 waves (>= 8 MiB of results each) so the D2H of
-    // wave w overlaps the kernels of wave w+1 instead of trailing one monolithic launch.
-    if (!cx.full_window || cx.host_args) {
-        const uint64_t bytes_per_task = std::max<uint64_t>(R, cx.host_args ? d.arg_stride : 0);
-        // a wave must carry enough kernel time to hide its launches: 8 MiB of byte results is ~22 us of
-        // pi dispatch; a byte of bit-packed results stands for 8 tasks, so 1 MiB is the same work
-        uint64_t min_wave_bytes = body.result_kind == FBR_RES_BITS8 ? (1ull << 20) : (8ull << 20);
-        if (const char* e = getenv("FBR_MIN_WAVE_KB")) min_wave_bytes = std::max<uint64_t>(4096, (uint64_t)atoll(e) << 10);   // tuning knob
-        const uint64_t min_wave_tasks = round_up(std::max<uint64_t>(1, min_wave_bytes / bytes_per_task), unit);
-        // 8 waves for ~100 MB maps, up to 64 for multi-GB ones (~64 MiB per wave): the first wave's
-        // H2D and the last wave's D2H are the only copies nothing overlaps with
-        uint64_t n_waves = std::min<uint64_t>(64, std::max<uint64_t>(8, part.count * bytes_per_task / (64ull << 20)));
-        // small outputs (bit-packed bools): per-copy set-up weighs more: T_kernel/n + n * 8 us is flattest at n = 5..6
-        if (body.result_kind == FBR_RES_BITS8 && !cx.host_args) n_waves = 6;
-        if (const char* e = getenv("FBR_WAVES")) n_waves = std::max<uint64_t>(1, (uint64_t)atoll(e));                          // tuning knob
-        const uint64_t share = round_up((part.count + n_waves - 1) / n_waves, unit);
-        static const bool pyr = getenv("FBR_PYRAMID") && atoi(getenv("FBR_PYRAMID")) != 0;
-        if (!(pyr && (cx.peer_push || cx.peer_out)))      // (the pyramid schedule uses the whole staging half)
-            cx.wave_tasks_cap = std::min(cx.wave_tasks_cap, std::max(min_wave_tasks, share));
     }
 
     // staging
@@ -1090,55 +1095,16 @@ static int submit_part(fbr_pool* p, SeqState& st, SeqPart& part, const BodyEntry
         CK(cudaHostAlloc((void**)&part.h_lost, sizeof(LostUnit) * std::max<uint32_t>(1, part.lost_cap), cudaHostAllocPortable));
     }
 
-    if (d.flags & FBR_WANT_SUM) {
-        if (!(body.flags & FBR_BODY_SUMMABLE)) return fail(FBR_EINVAL, "body %s results cannot be summed", body.name.c_str());
-        cx.sum_kind = 1;   // the dispatch kernel folds sum(results) while they are in registers
-    }
-
-    // Wave schedule of a block whose results stream out (host segment or the root GPU): the chain of copy-outs is the
-    // critical path when a wave's copy takes longer than its kernel (12.5 MB of bit-packed pi results: 38 us per
-    // 1.56 MB D2H -- 30 us of transfer + ~8 us of set-up -- against 31 us of kernel).  Equal waves are the default.
-    // Measured and dropped (each extra wave costs more chain latency than the schedule saves): opening the block with
-    // a quarter-size and a half-size wave so the first copy starts earlier (FBR_RAMP=1: 0.374 vs 0.358 ms per
-    // 1e8-task map), halving the LAST waves to shrink the exposed tail copy (FBR_TAPER=1: 0.375 vs 0.357 ms).
-    static const bool taper_on = getenv("FBR_TAPER") && atoi(getenv("FBR_TAPER")) != 0;
-    static const bool ramp_on = getenv("FBR_RAMP") && atoi(getenv("FBR_RAMP")) != 0;
-    const bool streaming_out = !cx.full_window && !cx.host_args;
-    const bool taper = taper_on && streaming_out;
-    const bool ramp = ramp_on && streaming_out && part.count > 4 * cx.wave_tasks_cap;
-    const uint64_t min_tail_tasks = round_up(std::max<uint64_t>(1, (256ull << 10) / std::max<uint32_t>(1, R)), unit);
-    // Blocks streamed over NVLink by copy engines (root-resident maps).  Raw peer copies reach 764 GB/s each way in one
-    // piece and 613 GB/s in 64 MB pieces (profiles/r02_peer_copy.txt), which suggested a pyramid of waves -- doubling
-    // from cap/16 up to the staging capacity, halving again towards the end: few large copies, short fill and drain.
-    // Measured on 2 GPUs (profiles/r02_peer_sweep.txt): 3.47 ms against 3.38 (equal 256 MB waves) and 3.27-3.41 (equal
-    // 64 MB waves) -- no gain, so equal waves stay the default (FBR_PYRAMID=1 enables the pyramid).
-    static const bool pyramid_on = getenv("FBR_PYRAMID") && atoi(getenv("FBR_PYRAMID")) != 0;
-    const bool pyramid = pyramid_on && (cx.peer_push || cx.peer_out);
-    const uint64_t pyr_base = round_up(std::max<uint64_t>(unit, cx.wave_tasks_cap / 16), unit);
-    uint64_t done_tasks = 0;
-    uint32_t wave_idx = 0;
-    while (done_tasks < part.count) {
-        uint64_t wt = std::min<uint64_t>(cx.wave_tasks_cap, part.count - done_tasks);
-        const uint64_t left = part.count - done_tasks;
-        if (ramp && wave_idx < 2) wt = std::min(left, round_up(cx.wave_tasks_cap >> (2 - wave_idx), unit));
-        if (pyramid) {
-            const uint64_t up = wave_idx < 8 ? pyr_base << wave_idx : cx.wave_tasks_cap;
-            const uint64_t down = std::max(pyr_base, round_up(left / 2, unit));
-            wt = std::min(std::min(left, cx.wave_tasks_cap), std::min(up, down));
-        }
-        ++wave_idx;
-        if (taper && left <= 2 * cx.wave_tasks_cap && left > min_tail_tasks)
-            wt = std::min(left, std::max(min_tail_tasks, round_up(left / 2, unit)));
+    // Equal waves of wave_tasks_cap tasks.  Task records go through the pinned ring window only when they are not an
+    // arithmetic progression the kernels can compute (shuffled arrival).  (The host may not overwrite a window whose
+    // previous H2D is in flight.)
+    const bool have_records = (d.flags & FBR_SHUFFLE) != 0;
+    for (uint64_t done_tasks = 0; done_tasks < part.count;) {
+        const uint64_t wt = std::min<uint64_t>(cx.wave_tasks_cap, part.count - done_tasks);
         const uint32_t n_units = (uint32_t)((wt + unit - 1) / unit);
         const uint64_t wno = w.wave_no++;
         const int rw = (int)(wno % kRecWindows);
         const uint64_t wave_first = part.first + done_tasks;  // map index of the wave's first task
-
-        // Task records go through the pinned ring window only when they are not an arithmetic
-        // progression the kernels can compute (shuffled arrival), or when FBR_RECORDS=1 asks for the
-        // explicit-record path.  (The host may not overwrite a window whose previous H2D is in flight.)
-        static const bool env_records = getenv("FBR_RECORDS") && atoi(getenv("FBR_RECORDS")) != 0;
-        const bool have_records = (d.flags & FBR_SHUFFLE) || env_records;
         if (have_records) {
             CK(cudaEventSynchronize(w.ev_rec_h2d[rw]));
             TaskRecord* hrec = w.h_records + (size_t)rw * kRecCapacity;
@@ -1152,7 +1118,7 @@ static int submit_part(fbr_pool* p, SeqState& st, SeqPart& part, const BodyEntry
                 r.func_id = (uint32_t)st.func_id;
                 r.attempt = part.attempt;
             }
-            if (d.flags & FBR_SHUFFLE) shuffle_records(hrec, n_units, d.shuffle_seed ^ (wno * 0x9E3779B97F4A7C15ull));
+            shuffle_records(hrec, n_units, d.shuffle_seed ^ (wno * 0x9E3779B97F4A7C15ull));
         }
         int rc = run_wave(p, st, part, body, n_units, wave_first, wt, true, have_records, wno);
         if (rc != FBR_OK) return rc;
@@ -1230,13 +1196,9 @@ static void cut_blocks(fbr_pool* p, const BodyEntry& body, const fbr_map_desc_t&
                        const std::vector<int>& workers, uint32_t attempt, std::vector<SeqPart>& out) {
     const int nw = (int)workers.size();
     if (nw == 0 || count == 0) return;
-    const uint32_t cs = d.chunksize ? d.chunksize : 32u;
-    const uint32_t unit = pick_unit(body, cs, (count + nw - 1) / nw, p->workers[workers[0]].sm_count, p->ring_bytes);
-    const uint64_t units_total = (count + unit - 1) / unit;
-    const uint64_t units_per = (units_total + nw - 1) / nw;
     for (int i = 0; i < nw; ++i) {
-        const uint64_t b0 = std::min<uint64_t>(count, (uint64_t)i * units_per * unit);
-        const uint64_t b1 = std::min<uint64_t>(count, (uint64_t)(i + 1) * units_per * unit);
+        uint64_t b0, b1;
+        block_range(body, d.chunksize, count, nw, i, p->workers[workers[0]].sm_count, p->ring_bytes, &b0, &b1);
         if (b1 <= b0) continue;
         SeqPart part;
         part.worker = workers[i];
@@ -1457,20 +1419,43 @@ int fbr_plan_query(int func_id, uint64_t n_tasks, uint32_t chunksize, uint64_t r
     if (!plan || !body_of(func_id) || n_workers < 1 || worker < 0 || worker >= n_workers)
         return fail(FBR_EINVAL, "bad arguments");
     const BodyEntry& body = *body_of(func_id);
-    const uint64_t ring = round_up(ring_bytes ? ring_bytes : (256ull << 20), 4096);
-    const uint32_t cs = chunksize ? chunksize : 32u;
+    const uint64_t ring = pool_ring_bytes(ring_bytes);
     if (sm_count <= 0) sm_count = 148;
-    // the same two steps fbr_map_submit takes: blocks on the map-level unit, then the block's own unit
-    const uint32_t unit = pick_unit(body, cs, (n_tasks + n_workers - 1) / n_workers, sm_count, ring);
-    const uint64_t units_total = (n_tasks + unit - 1) / unit;
-    const uint64_t units_per = (units_total + n_workers - 1) / n_workers;
-    const uint64_t b0 = std::min<uint64_t>(n_tasks, (uint64_t)worker * units_per * unit);
-    const uint64_t b1 = std::min<uint64_t>(n_tasks, (uint64_t)(worker + 1) * units_per * unit);
+    // the same two steps fbr_map_submit takes: blocks on the map-level unit (cut_blocks), then the block's own unit
+    // (plan_part)
+    uint64_t b0, b1;
+    block_range(body, chunksize, n_tasks, n_workers, worker, sm_count, ring, &b0, &b1);
     plan->block_first = b0;
     plan->block_count = b1 - b0;
-    plan->unit_tasks = pick_unit(body, cs, b1 - b0, sm_count, ring);
+    plan->unit_tasks = pick_unit(body, chunksize, b1 - b0, sm_count, ring);
     plan->slot_stride = (uint32_t)round_up((uint64_t)plan->unit_tasks * body.result_bytes, 16);
     plan->n_units = plan->block_count ? (plan->block_count + plan->unit_tasks - 1) / plan->unit_tasks : 0;
+    return FBR_OK;
+}
+
+// What plan_part decides for the block [first, first + count) of map `d` on worker `worker` of a pool with `ring_bytes`
+// (0: the default) and `pool_flags`, on a device with `sm_count` SMs (<= 0: 148): the claim unit, the slot stride, the
+// path flags (bit k set = the k-th of args_dev, out_dev, keep_on_device, resilient, peer_out, peer_push, zero_copy,
+// full_window, host_args, overlap, direct), the tasks per wave and the number of waves.  Needs no device, so the
+// schedule can be tested anywhere.  (Internal: not part of the public header.)
+int fbr_internal_plan_part(const fbr_map_desc_t* d, uint64_t first, uint64_t count, int worker, int root_alive,
+                           int sm_count, uint64_t ring_bytes, uint32_t pool_flags, int has_out, uint32_t* unit_tasks,
+                           uint32_t* slot_stride, uint32_t* path_flags, uint64_t* wave_tasks_cap, uint64_t* n_waves) {
+    if (!d || !body_of(d->func_id) || count == 0 || worker < 0 || !unit_tasks || !slot_stride || !path_flags ||
+        !wave_tasks_cap || !n_waves)
+        return fail(FBR_EINVAL, "bad arguments");
+    PartPlan c;
+    const int rc = plan_part(*body_of(d->func_id), *d, first, count, worker, root_alive != 0, sm_count > 0 ? sm_count : 148,
+                             pool_ring_bytes(ring_bytes), pool_flags, has_out != 0, &c);
+    if (rc != FBR_OK) return rc;
+    const bool path[] = {c.args_dev, c.out_dev, c.keep_on_device, c.resilient, c.peer_out, c.peer_push,
+                         c.zero_copy, c.full_window, c.host_args, c.overlap, c.direct};
+    *path_flags = 0;
+    for (size_t k = 0; k < sizeof path / sizeof path[0]; ++k) *path_flags |= (uint32_t)path[k] << k;
+    *unit_tasks = c.unit;
+    *slot_stride = c.slot_stride;
+    *wave_tasks_cap = c.wave_tasks_cap;
+    *n_waves = (count + c.wave_tasks_cap - 1) / c.wave_tasks_cap;   // submit_part's loop: equal waves, a shorter last one
     return FBR_OK;
 }
 
@@ -1482,7 +1467,7 @@ int fbr_pool_create(int n_workers, const int* device_ids, uint64_t ring_bytes, u
     if (ndev == 0) return fail(FBR_ENODEV, "no CUDA device visible; fiber_b200 has no CPU fallback");
     std::unique_ptr<fbr_pool> p(new fbr_pool());
     p->flags = flags;
-    p->ring_bytes = round_up(ring_bytes ? ring_bytes : (256ull << 20), 4096);
+    p->ring_bytes = pool_ring_bytes(ring_bytes);
     if (p->ring_bytes >= (1ull << 35)) return fail(FBR_EINVAL, "ring_bytes must be below 32 GiB (32-bit vector index in gather_ordered)");
     memset(&p->stats, 0, sizeof p->stats);
     p->workers.resize(n_workers);
@@ -1562,7 +1547,6 @@ int fbr_pool_join(fbr_pool_t* p) {
         CK(cudaStreamSynchronize(w.s_comp));
         CK(cudaStreamSynchronize(w.s_gath));
         CK(cudaStreamSynchronize(w.s_out));
-        CK(cudaStreamSynchronize(w.s_out2));
     }
     return FBR_OK;
 }
@@ -1711,8 +1695,7 @@ int fbr_map_submit(fbr_pool_t* p, const fbr_map_desc_t* d, uint64_t* seq_out) {
             st->own_out = true;
         }
         int failed_worker = -1, rc = FBR_OK;
-        static const bool serial = getenv("FBR_SERIAL_SUBMIT") && atoi(getenv("FBR_SERIAL_SUBMIT")) != 0;
-        if (st->parts.size() > 1 && !serial) {
+        if (st->parts.size() > 1) {
             // one submit thread per worker (see SubmitThread); this thread holds the pool lock meanwhile
             if (p->submitters.size() < p->workers.size()) p->submitters.resize(p->workers.size());
             SeqState* stp = st.get();

@@ -1,5 +1,4 @@
-"""Pipelined pi steps with FBR_POOL_OVERLAP (gather(k) on a second stream while dispatch(k+1) runs); A/B the
-gather's CTA budget with FBR_GATHER_OCC."""
+"""Pipelined pi steps with FBR_POOL_OVERLAP (gather(k) on a second stream while dispatch(k+1) runs)."""
 import os
 import sys
 import time
@@ -18,6 +17,6 @@ t0 = time.perf_counter()
 seqs = [e2.submit("pi_inside_det", bench.PI_TASKS, o2) for _ in range(steps)]
 cnt = [e2.wait(q)[0] for q in seqs]
 dt = (time.perf_counter() - t0) / steps
-print("overlap gather_occ=%s  %.4f ms/step  count %d" % (os.environ.get("FBR_GATHER_OCC", "-"), dt * 1e3, cnt[-1]), flush=True)
+print("overlap  %.4f ms/step  count %d" % (dt * 1e3, cnt[-1]), flush=True)
 e2.dfree(o2)
 e2.close()

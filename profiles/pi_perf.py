@@ -1,4 +1,4 @@
-"""Event-timed pi dispatch / gather kernels only (quick A/B of FBR_DISPATCH_OCC / FBR_UNIT_TASKS).
+"""Event-timed pi dispatch / gather kernels only.
 
     python profiles/pi_perf.py [steps] [pi_inside_det|pi_inside_bits8]
 """
@@ -20,8 +20,7 @@ for i in range(steps + 3):
         eng.stats(reset=True)
     cnt = eng.wait(eng.submit(body, n, out))[0]
 st = eng.stats()
-print("%s occ=%s unit=%s  dispatch %.4f ms  gather %.4f ms  count %d" % (
-    body, os.environ.get("FBR_DISPATCH_OCC", "-"), os.environ.get("FBR_UNIT_TASKS", "-"),
-    st["dispatch_ms"] / st["dispatch_launches"], st["gather_ms"] / max(1, st["gather_launches"]), cnt), flush=True)   # direct placement: no gather
+print("%s  dispatch %.4f ms  gather %.4f ms  count %d" % (
+    body, st["dispatch_ms"] / st["dispatch_launches"], st["gather_ms"] / max(1, st["gather_launches"]), cnt), flush=True)   # direct placement: no gather
 eng.dfree(out)
 eng.close()
