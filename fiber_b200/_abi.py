@@ -19,6 +19,7 @@ FBR_OK, FBR_EINVAL, FBR_ECUDA, FBR_ENOMEM, FBR_ESTATE, FBR_ETIMEOUT, FBR_ETASK, 
 FBR_RES_BYTES, FBR_RES_BOOL, FBR_RES_I64, FBR_RES_U32, FBR_RES_F64X2, FBR_RES_NONE, FBR_RES_BITS8 = range(7)
 # body flags
 FBR_BODY_INDEX_ARG, FBR_BODY_NEEDS_SHARED, FBR_BODY_SUMMABLE, FBR_BODY_INDEX_ONLY = 0x1, 0x2, 0x4, 0x8
+FBR_BODY_RECORD = 0x10
 # pool flags
 FBR_POOL_TIMING, FBR_POOL_OVERLAP = 0x1, 0x2
 # map flags

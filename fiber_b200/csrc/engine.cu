@@ -27,6 +27,7 @@
 #include <deque>
 #include <memory>
 #include <mutex>
+#include <numeric>
 #include <string>
 #include <thread>
 #include <unordered_map>
@@ -613,8 +614,9 @@ static void worker_destroy(Worker& w) {
 }
 
 // Claim-unit size: near the body's preferred size, a multiple of the API chunksize when the chunk
-// is smaller (so chunk boundaries coincide with unit boundaries), and a multiple of 16/R tasks so
-// every full slot is 16 B aligned on both sides of the gather.  `chunksize` 0 stands for the default, 32.
+// is smaller (so chunk boundaries coincide with unit boundaries), and a multiple of 16/gcd(R, 16) tasks so
+// every full slot is 16 B aligned on both sides of the gather (R = 12: units of 4k tasks).  `chunksize` 0 stands for
+// the default, 32.
 static uint32_t pick_unit(const BodyEntry& b, uint32_t chunksize, uint64_t n_tasks, int sm_count, uint64_t ring_bytes) {
     uint32_t pref = b.unit_tasks;
     if (pref == 1) return 1;
@@ -624,7 +626,7 @@ static uint32_t pick_unit(const BodyEntry& b, uint32_t chunksize, uint64_t n_tas
     while (pref > 1 && (uint64_t)pref * per_task > ring_bytes / 2) pref >>= 1;
     // small maps: shrink the unit so the work still spreads over the SMs
     while (pref > 256 && (uint64_t)pref * (uint64_t)sm_count > n_tasks) pref >>= 1;
-    const uint32_t align = b.result_bytes < 16 ? 16u / b.result_bytes : 1u;
+    const uint32_t align = 16u / std::gcd(b.result_bytes, 16u);
     uint32_t unit = pref;
     if (chunksize <= pref) {
         uint32_t m = chunksize;  // lcm(chunksize, align)
@@ -1390,7 +1392,20 @@ int fbr_register_body(const char* name, const char* module_path, const char* ent
         dlclose(h);
         return fail(FBR_EINVAL, "module %s exports body '%s', not '%s'", module_path, m->name, name);
     }
-    if (m->result_bytes == 0 || m->unit_tasks == 0 || (m->arg_bytes % 8) != 0 || m->result_kind > FBR_RES_BITS8) {
+    if (m->flags & FBR_BODY_RECORD) {
+        // record bodies (dispatch_record_kernel): 4..256-byte records in whole words, explicit arguments, opaque results
+        auto bad = [](uint32_t b) { return b < 4 || b > 256 || b % 4 != 0; };
+        if (bad(m->arg_bytes) || bad(m->result_bytes) || m->unit_tasks == 0 || m->result_kind != FBR_RES_BYTES) {
+            dlclose(h);
+            return fail(FBR_EINVAL, "module %s: record body '%s' needs argument and result records of 4..256 bytes in whole "
+                        "words (got %u / %u) and result kind FBR_RES_BYTES", module_path, name, m->arg_bytes, m->result_bytes);
+        }
+        if (m->flags & (FBR_BODY_SUMMABLE | FBR_BODY_INDEX_ARG | FBR_BODY_INDEX_ONLY | FBR_BODY_NEEDS_SHARED)) {
+            dlclose(h);
+            return fail(FBR_EINVAL, "module %s: record body '%s' cannot be summable, take range() indices or a shared block",
+                        module_path, name);
+        }
+    } else if (m->result_bytes == 0 || m->unit_tasks == 0 || (m->arg_bytes % 8) != 0 || m->result_kind > FBR_RES_BITS8) {
         dlclose(h);
         return fail(FBR_EINVAL, "module %s: body '%s' has an invalid record layout", module_path, name);
     }
@@ -1621,6 +1636,12 @@ int fbr_map_submit(fbr_pool_t* p, const fbr_map_desc_t* d, uint64_t* seq_out) {
             return fail(FBR_EINVAL, "body %s needs explicit argument records (arg_stride=0)", body.name.c_str());
     } else if (body.flags & FBR_BODY_INDEX_ONLY) {
         return fail(FBR_EINVAL, "body %s takes range() arguments only (arg_stride must be 0)", body.name.c_str());
+    } else if (body.flags & FBR_BODY_RECORD) {
+        // the record kernel copies whole words from any 4-byte aligned record (kernels.cuh, dispatch_record_kernel)
+        if (d->arg_stride < body.arg_bytes || (d->arg_stride % 4) != 0)
+            return fail(FBR_EINVAL, "arg_stride %u invalid for body %s (arg_bytes %u)", d->arg_stride, body.name.c_str(), body.arg_bytes);
+        if (d->n_tasks && !d->args) return fail(FBR_EINVAL, "args is NULL");
+        if ((uintptr_t)d->args % 4) return fail(FBR_EINVAL, "argument records of body %s must be 4-byte aligned", body.name.c_str());
     } else {
         if (d->arg_stride < body.arg_bytes || (d->arg_stride % 8) != 0)
             return fail(FBR_EINVAL, "arg_stride %u invalid for body %s (arg_bytes %u)", d->arg_stride, body.name.c_str(), body.arg_bytes);

@@ -906,6 +906,143 @@ __global__ void __launch_bounds__(160) dispatch_payload_map_tma_kernel(const Wav
 }
 
 // ================================================================================================
+// dispatch: record body -- a ThreadBody whose Arg and Res are trivially copyable records of 4..256 bytes
+// (multiples of 4): floats, small structs, packed float3 points.  Explicit argument records only.
+// A CTA stages each tile of its unit through shared memory:
+//   1. cp.async copies the tile's argument words into an IN stage (one warp instruction = 128 consecutive
+//      bytes of the wave's arguments, whatever the record size or alignment);
+//   2. thread i runs B::run on record i of the stage and writes its Res into the OUT tile;
+//   3. the CTA stores the OUT tile to the slot, one warp instruction = 128 consecutive bytes.
+// The copy of tile k+1 is in flight while tile k computes (two IN stages).  Records sit in shared memory at an
+// odd number of words apart, so the per-thread record reads and result writes are free of bank conflicts for
+// every record size (a 64 B record at its natural stride would be a 16-way conflict).  Record bases need only be
+// 4-byte aligned: an arg_stride of 12 at an odd record offset, a unit whose result bytes end mid-vector and the
+// argument records of a strided layout (arg_stride > sizeof(Arg)) all take the same word path.
+// Algorithmic bytes per task: sizeof(Arg) read + sizeof(Res) written.
+// ================================================================================================
+namespace rec {
+__device__ __forceinline__ void cp_async4(void* s, const void* g) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((uint32_t)__cvta_generic_to_shared(s)), "l"(g) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+constexpr uint32_t kStageBytes = 12288;     // shared memory of one IN stage (OUT tile: at most the same)
+constexpr uint32_t odd_words(uint32_t bytes) { return (bytes / 4) | 1u; }   // padded record pitch in words
+
+template <class B>
+struct Layout {
+    using Arg = typename B::Arg;
+    using Res = typename B::Res;
+    static constexpr uint32_t kArgWords = sizeof(Arg) / 4, kResWords = sizeof(Res) / 4;
+    static constexpr uint32_t kArgPitch = odd_words(sizeof(Arg)), kResPitch = odd_words(sizeof(Res));   // words
+    static constexpr uint32_t kMaxPitch = kArgPitch > kResPitch ? kArgPitch : kResPitch;
+    static constexpr uint32_t kTasks = (kStageBytes / 4 / kMaxPitch) < 2048u ? (kStageBytes / 4 / kMaxPitch) : 2048u;   // per tile
+    static constexpr uint32_t kInWords = kTasks * kArgPitch, kOutWords = kTasks * kResPitch;
+    static_assert(std::is_trivially_copyable<Arg>::value && std::is_trivially_copyable<Res>::value,
+                  "record bodies take and return trivially copyable records");
+    static_assert(sizeof(Arg) % 4 == 0 && sizeof(Arg) >= 4 && sizeof(Arg) <= 256, "sizeof(Arg) must be a multiple of 4 in [4, 256]");
+    static_assert(sizeof(Res) % 4 == 0 && sizeof(Res) >= 4 && sizeof(Res) <= 256, "sizeof(Res) must be a multiple of 4 in [4, 256]");
+    static_assert((2 * kInWords + kOutWords) * 4 <= 48 * 1024, "static shared memory of the record kernel");
+};
+
+// Copy the argument words of tasks [0, cnt) of a tile (records `stride` bytes apart from `src`) into `stage`.
+template <class L>
+__device__ __forceinline__ void load_tile(uint32_t* stage, const uint8_t* src, uint32_t stride, uint32_t cnt) {
+    const uint32_t total = cnt * L::kArgWords;
+    for (uint32_t w = threadIdx.x; w < total; w += kThreads) {
+        const uint32_t r = w / L::kArgWords, j = w - r * L::kArgWords;
+        cp_async4(stage + r * L::kArgPitch + j, src + (size_t)r * stride + 4u * j);
+    }
+}
+}  // namespace rec
+
+template <class B>
+__global__ void __launch_bounds__(kThreads) dispatch_record_kernel(const WaveParams wp) {
+    using L = rec::Layout<B>;
+    using Arg = typename B::Arg;
+    using Res = typename B::Res;
+    __shared__ uint32_t s_in[2 * L::kInWords];
+    __shared__ uint32_t s_out[L::kOutWords];
+    __shared__ uint32_t s_ticket[2];
+    __shared__ int s_fault;
+    if (threadIdx.x == 0) s_fault = 0;
+    const ErrSink es{wp.err_word, &s_fault};
+    TicketClaimer tc{wp.ticket, 0u};
+    tc.prime();
+    uint32_t iter = 0;
+    uint32_t t = tc.claim_db(s_ticket, iter++);
+    TaskRecord rc{};
+    if (t < wp.n_units) {
+        rc = wave_record(wp, t);
+        rec::load_tile<L>(s_in, wp.args + rc.arg_off, wp.arg_stride, min(rc.count, L::kTasks));
+    }
+    rec::cp_async_commit();
+    uint32_t tile = 0, buf = 0;
+    while (t < wp.n_units) {
+        // the tile to prefetch: the next one of this unit, or the first of the next unit claimed
+        uint32_t nt = t, ntile = tile + 1;
+        TaskRecord nrc = rc;
+        const bool last = (uint64_t)ntile * L::kTasks >= rc.count;
+        if (last) {
+            nt = tc.claim_db(s_ticket, iter++);
+            ntile = 0;
+            if (nt < wp.n_units) nrc = wave_record(wp, nt);
+        }
+        if (nt < wp.n_units) {
+            const uint32_t first = ntile * L::kTasks;
+            rec::load_tile<L>(s_in + (buf ^ 1u) * L::kInWords, wp.args + nrc.arg_off + (size_t)first * wp.arg_stride,
+                              wp.arg_stride, min(nrc.count - first, L::kTasks));
+        }
+        rec::cp_async_commit();
+        rec::cp_async_wait<1>();      // this thread's copies of the current tile have landed ...
+        __syncthreads();              // ... and everyone else's; the previous OUT tile has been stored
+
+        const uint32_t first = tile * L::kTasks;
+        const uint32_t cnt = min(rc.count - first, L::kTasks);
+        const uint32_t* in = s_in + buf * L::kInWords;
+        const uint64_t gidx0 = wp.index_base + rc.first + first;
+        for (uint32_t i = threadIdx.x; i < cnt; i += kThreads) {
+            uint32_t aw[L::kArgWords];
+#pragma unroll
+            for (uint32_t k = 0; k < L::kArgWords; ++k) aw[k] = in[i * L::kArgPitch + k];
+            Arg a;
+            memcpy(&a, aw, sizeof(Arg));
+            const Res r = B::run(a, gidx0 + i, es, rc.attempt);
+            uint32_t rw[L::kResWords];
+            memcpy(rw, &r, sizeof(Res));
+#pragma unroll
+            for (uint32_t k = 0; k < L::kResWords; ++k) s_out[i * L::kResPitch + k] = rw[k];
+        }
+        __syncthreads();              // OUT tile complete, fault reports of the tile are in, IN stage `buf` is free
+
+        uint32_t* dst = reinterpret_cast<uint32_t*>(wp.ring + (size_t)t * wp.slot_stride + (size_t)first * sizeof(Res));
+        const uint32_t total = cnt * L::kResWords;
+        for (uint32_t w = threadIdx.x; w < total; w += kThreads) {
+            const uint32_t r = w / L::kResWords, j = w - r * L::kResWords;
+            dst[w] = s_out[r * L::kResPitch + j];
+        }
+        if (last && threadIdx.x == 0) {
+            bool lost = false;
+            if constexpr (B::kCanFault) {
+                lost = s_fault != 0;  // every report of this unit happened before the barrier above
+                s_fault = 0;          // the next unit computes only after the next barrier
+                if (lost && !wp.resilient)
+                    atomicMin(wp.err_word, (unsigned long long)(((wp.index_base + rc.first) << 8) | TASK_FAULT));
+            }
+            put_header(wp, t, SlotHeader{rc.seq, rc.count | ((lost && wp.resilient) ? kUnitLost : 0u), rc.first});
+        }
+        t = nt;
+        rc = nrc;
+        tile = ntile;
+        buf ^= 1u;
+    }
+    rec::cp_async_wait<0>();
+    tc.rearm(wp.n_units);
+}
+
+// ================================================================================================
 // payload_fill: w[t][j] = low32(splitmix64(SEED ^ (t*1024 + j))); each thread emits 16 B.
 // ================================================================================================
 __global__ void __launch_bounds__(kThreads) payload_fill_kernel(uint4* out, uint64_t t0, uint64_t n_vec) {

@@ -196,6 +196,9 @@ class ResultArray(collections.abc.Sequence):
     def sum(self):
         if self._sum is not None:
             return self._sum
+        py_sum = getattr(self._spec, "py_sum", None)
+        if py_sum is not None:          # record bodies: the builtin's sum of the list (floats left to right, tuples raise)
+            return py_sum(self)
         if self._bits is not None:
             return int(np.unpackbits(self._bits).sum())   # the bits past n are zero
         if self._a.dtype.kind in "iu" and self._a.dtype.itemsize == 8:

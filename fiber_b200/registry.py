@@ -21,7 +21,7 @@ from . import _abi
 _BOUND = {}  # callables that cannot carry attributes (builtins) -> body name
 
 
-def device_body(name, source=None, entry="fbr_body_entry", args="i64", bits_entry=None, **meta):
+def device_body(name, source=None, entry="fbr_body_entry", args="i64", bits_entry=None, result=None, **meta):
     """Decorator: ``@device_body("pi_inside_det")`` binds ``func`` to the device body ``name`` and sets
     ``func.__fiber_meta__`` (``gpu=1`` unless overridden), like ``fiber.meta``.
 
@@ -33,7 +33,14 @@ def device_body(name, source=None, entry="fbr_body_entry", args="i64", bits_entr
     how a callable that is not compiled into libfiber_b200 gets its device code there.  ``args`` names the
     argument record layout: ``"i64"`` (one int) or ``"i64x2"`` (two ints).  A bool body may also export its
     bit-packed twin (``FBR_EXPORT_BOOL_BODY_BITS(Body, "<name>_bits8", <bits_entry>, flags)``): pass ``bits_entry``
-    and its results travel one bit each, like the compiled-in bool body's."""
+    and its results travel one bit each, like the compiled-in bool body's.
+
+    A body of floats or small structs (``FBR_EXPORT_RECORD_BODY``) declares its records as NumPy dtypes:
+    ``args=`` and ``result=`` take anything ``np.dtype()`` accepts -- ``"f8"``, ``"<f4"``, ``"i4"``, ``"3f4"`` (a packed
+    float3) or a structured list of named fields -- and must match the module's ``arg_bytes`` / ``result_bytes``.
+    Its tasks are encoded as records (``map``: one record per item, NumPy arrays of the record layout without a copy;
+    ``starmap`` / ``apply``: the positional arguments are the fields in order, keywords name them) and its results
+    decode to Python floats / ints, or tuples for multi-field records."""
     from .meta import VALID_META_KEYS
     for k in meta:
         assert k in VALID_META_KEYS, "Invalid meta argument \"{}\"".format(k)
@@ -41,7 +48,7 @@ def device_body(name, source=None, entry="fbr_body_entry", args="i64", bits_entr
     md.update(meta)
     if source is not None:
         from . import bodies
-        register_module(name, bodies.compile_module(name, source), entry, args, bits_entry)
+        register_module(name, bodies.compile_module(name, source), entry, args, bits_entry, result)
 
     def decorator(func):
         bind(func, name, **md)
@@ -49,7 +56,8 @@ def device_body(name, source=None, entry="fbr_body_entry", args="i64", bits_entr
     return decorator
 
 
-_MODULES = {}   # body name -> (module path, entry, argument layout) of bodies registered from their own module
+_MODULES = {}   # body name -> (module path, entry, argument layout, bits entry, result layout) of bodies registered
+                # from their own module
 
 
 def module_of(name):
@@ -57,24 +65,32 @@ def module_of(name):
     return _MODULES.get(name)
 
 
-def register_module(name, module_path, entry="fbr_body_entry", args="i64", bits_entry=None):
+def register_module(name, module_path, entry="fbr_body_entry", args="i64", bits_entry=None, result=None):
     """``fbr_register_body`` + the host-side encoder for the body's argument records (and, with ``bits_entry``, the
-    body's bit-packed twin ``<name>_bits8``)."""
+    body's bit-packed twin ``<name>_bits8``).  ``args`` is ``"i64"``, ``"i64x2"`` or ``"bits8"``, or -- with ``result``,
+    and always for a record body (``FBR_BODY_RECORD``) -- a NumPy dtype of the argument record (see ``device_body``)."""
     import ctypes
-    _MODULES[name] = (str(module_path), entry, args, bits_entry)
+    _MODULES[name] = (str(module_path), entry, args, bits_entry, result)
     if bits_entry is not None:
         twin = name + "_bits8"
         register_module(twin, module_path, bits_entry, "bits8")
         _MODULES.pop(twin, None)
         BITS_TWIN[name] = twin
     L = _abi.load()
+    specs = _load_specs()      # before the body joins the engine's table: it is not listed as a plain BodySpec
     fid = ctypes.c_int(-1)
     _abi.check(L.fbr_register_body(name.encode(), str(module_path).encode(), entry.encode(), ctypes.byref(fid)))
-    specs = _load_specs()
     if name not in specs:
         info = _abi.BodyInfo()
         _abi.check(L.fbr_body_info(fid.value, ctypes.byref(info)))
-        if args == "i64":
+        legacy = isinstance(args, str) and args in ("i64", "i64x2", "bits8")
+        if result is not None or not legacy or (info.flags & _abi.FBR_BODY_RECORD):
+            try:
+                specs[name] = _Record(info, args, result)
+            except (TypeError, ValueError):
+                _MODULES.pop(name, None)
+                raise
+        elif args == "i64":
             specs[name] = _UnaryI64(info)
         elif args == "i64x2":
             specs[name] = _BinaryI64(info)
@@ -445,6 +461,146 @@ class _Parzen(BodySpec):
         enc = Encoded(len(a), args=a, arg_stride=8)
         enc.shared = self.shared_block(*first) if first is not None else None
         return enc
+
+
+def _record_dtype(layout, what):
+    """NumPy dtype of a record layout: anything ``np.dtype()`` takes, plus the names of the integer layouts."""
+    if isinstance(layout, str) and layout in ("i64", "i64x2"):
+        layout = "<i8" if layout == "i64" else "2<i8"
+    try:
+        return np.dtype(layout)
+    except TypeError as e:
+        raise ValueError("%s: %r is not a NumPy dtype (%s)" % (what, layout, e)) from None
+
+
+def _leaves(dt, off=0):
+    """(byte offset, scalar dtype) of every scalar of record dtype ``dt``, in memory order."""
+    if dt.names:
+        for n in dt.names:
+            f, o = dt.fields[n][:2]
+            yield from _leaves(f, off + o)
+    elif dt.subdtype is not None:
+        base, shape = dt.subdtype
+        for i in range(int(np.prod(shape))):
+            yield from _leaves(base, off + i * base.itemsize)
+    else:
+        yield off, dt
+
+
+_MISSING = object()
+
+
+class _Record(BodySpec):
+    """A body whose argument and result records are NumPy dtypes (out-of-tree record bodies,
+    ``FBR_EXPORT_RECORD_BODY``): ``f(x)`` of a scalar dtype, ``f(x, y, z)`` of a structured dtype's fields (or of the
+    elements of a sub-array dtype such as ``"3f4"``).  The call rules follow the reference's task tuple
+    (fiber/pool.py:803-821): ``map`` passes each item as the one argument -- a number, the value of a one-field record,
+    or the tuple of field values --
+    ``starmap`` its items as positional arguments, ``apply`` positional arguments then keywords by field name."""
+
+    def __init__(self, info, args, result):
+        super().__init__(info)
+        if result is None:
+            raise ValueError("%s: a record body needs result=<dtype> of its %d-byte result record" % (self.name, info.result_bytes))
+        self.arg_dtype = _record_dtype(args, "%s args" % self.name)
+        self.res_dtype = _record_dtype(result, "%s result" % self.name)
+        for what, dt, nb in (("argument", self.arg_dtype, self.arg_bytes), ("result", self.res_dtype, self.result_bytes)):
+            if dt.itemsize != nb:
+                raise ValueError("%s: %s dtype %s has %d bytes, the module's %s record has %d"
+                                 % (self.name, what, dt, dt.itemsize, what, nb))
+        dt = self.arg_dtype
+        self.fields = dt.names                      # keyword names (structured dtypes only)
+        self.arity = len(dt.names) if dt.names else (int(np.prod(dt.subdtype[1])) if dt.subdtype is not None else 1)
+        self._leaves = list(_leaves(dt))
+
+    # ---- arguments ------------------------------------------------------------------------------
+    def _row(self, args, kwds):
+        """Positional arguments, then keywords by field name -> the record's field values in order."""
+        n = self.arity
+        if len(args) > n:
+            raise TypeError("%s() takes %d positional argument%s but %d were given" % (self.name, n, "s" * (n != 1), len(args)))
+        vals = list(args) + [_MISSING] * (n - len(args))
+        for k, v in kwds.items():
+            if not self.fields or k not in self.fields:
+                raise TypeError("%s() got an unexpected keyword argument %r" % (self.name, k))
+            i = self.fields.index(k)
+            if vals[i] is not _MISSING:
+                raise TypeError("%s() got multiple values for argument %r" % (self.name, k))
+            vals[i] = v
+        if any(v is _MISSING for v in vals):
+            missing = [self.fields[i] if self.fields else str(i) for i, v in enumerate(vals) if v is _MISSING]
+            raise TypeError("%s() missing required argument(s): %s" % (self.name, ", ".join(missing)))
+        return vals
+
+    def _records(self, rows):
+        dt = self.arg_dtype
+        if dt.names:
+            return np.array([tuple(r) for r in rows], dtype=dt)
+        if dt.subdtype is not None:
+            base, shape = dt.subdtype
+            return np.array(rows, dtype=base).reshape((len(rows),) + shape)
+        return np.array([r[0] for r in rows], dtype=dt)
+
+    def _array_records(self, a):
+        """A NumPy array as argument records: itself when its rows already are the record layout (no copy)."""
+        dt = self.arg_dtype
+        if a.ndim == 1 and a.dtype == dt:
+            return np.ascontiguousarray(a)
+        if a.ndim == 2 and a.shape[1] == len(self._leaves) and a.shape[1] * a.itemsize == dt.itemsize and \
+                all(b == a.dtype and off == i * a.itemsize for i, (off, b) in enumerate(self._leaves)):
+            return np.ascontiguousarray(a)          # (n, k) rows of the record's k scalars
+        if a.ndim == 1 and not dt.names and dt.subdtype is None and a.dtype.kind in "biuf":
+            return np.ascontiguousarray(a, dtype=dt)
+        if dt.names and a.dtype.names == dt.names and a.ndim == 1:
+            return a.astype(dt)
+        raise TypeError("%s: an array of dtype %s and shape %s does not hold %s records" % (self.name, a.dtype, a.shape, dt))
+
+    def _fast_map_ok(self, items):
+        return True
+
+    def _encode(self, items, fast, apply=False):
+        if fast:
+            if isinstance(items, np.ndarray):
+                a = self._array_records(items)
+            elif self.arity == 1 and not self.fields and self.arg_dtype.subdtype is None:
+                a = np.array(items if isinstance(items, list) else list(items), dtype=self.arg_dtype)
+            elif self.arity == 1:
+                a = self._records([(it,) for it in items])      # one field: the item is its value, f(item)
+            else:
+                rows = []
+                for it in items:
+                    if not isinstance(it, (tuple, list, np.ndarray, np.void)):
+                        raise TypeError("%s: map() items must be tuples of the %d record fields, got %r" % (self.name, self.arity, it))
+                    rows.append(self._row(tuple(it), {}))
+                a = self._records(rows)
+        else:
+            a = self._records([self._row(*self._split(it, apply)) for it in items])
+        return Encoded(len(a), args=a, arg_stride=self.arg_dtype.itemsize)
+
+    # ---- results --------------------------------------------------------------------------------
+    def result_dtype(self):
+        dt = self.res_dtype
+        if dt.subdtype is not None:
+            return dt.subdtype[0], dt.subdtype[1]
+        return dt, ()
+
+    def to_python(self, row):
+        if self.res_dtype.names or self.res_dtype.subdtype is not None:
+            return self.rows_to_list(np.asarray(row)[None])[0]
+        return row.item()
+
+    def rows_to_list(self, arr):
+        if self.res_dtype.subdtype is not None:
+            return [tuple(r) for r in arr.tolist()]
+        return arr.tolist()                          # structured rows: tuples of Python scalars
+
+    def unpack_result(self, raw):
+        return self.to_python(np.frombuffer(bytes(raw[:self.result_bytes]), dtype=self.res_dtype)[0])
+
+    def py_sum(self, values):
+        """``sum(results)`` exactly as the builtin computes it over the reference's list (the device does not fold
+        record results): floats added left to right, and TypeError for tuples."""
+        return sum(values.tolist())
 
 
 class _Payload4K(BodySpec):

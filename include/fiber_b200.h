@@ -67,6 +67,9 @@ typedef enum fbr_result_kind {
 #define FBR_BODY_NEEDS_SHARED 0x2u /* body reads a shared (broadcast) argument block */
 #define FBR_BODY_SUMMABLE 0x4u    /* the dispatch kernel can fold sum(results) (bool/int64/u32; popcount for bits) */
 #define FBR_BODY_INDEX_ONLY 0x8u  /* body takes range() arguments only (arg_stride must be 0) */
+#define FBR_BODY_RECORD 0x10u     /* record body (FBR_EXPORT_RECORD_BODY): argument and result records of 4..256 bytes,
+                                     multiples of 4 (result_kind FBR_RES_BYTES); explicit, 4-byte aligned argument
+                                     records only (arg_stride % 4 == 0); not summable, no range() or shared block */
 
 typedef struct fbr_body_info {
     int32_t func_id;
@@ -86,7 +89,8 @@ int fbr_body_lookup(const char* name, int* func_id);
  * (fiber/pool.py:961) and the worker calls it (fiber/pool.py:806,809,820); here the callable's device
  * code may be compiled separately from this library: a shared object built with nvcc for sm_100a from a
  * source that includes include/fiber_b200_body.cuh, defines a ThreadBody struct and exports it with
- * FBR_EXPORT_THREAD_BODY(Body, name, entry).  fbr_register_body dlopen()s `module_path`, calls `entry`
+ * FBR_EXPORT_THREAD_BODY(Body, name, entry) (integer and bool results), or with FBR_EXPORT_RECORD_BODY(Body, name,
+ * entry, flags) for any float / struct argument and result records (FBR_BODY_RECORD).  fbr_register_body dlopen()s `module_path`, calls `entry`
  * to obtain the module descriptor below, checks its ABI stamp and appends the body to the table
  * (func_id >= the compiled-in count; the same name may be registered once).  The module's launch routine
  * receives the same wave parameters as the compiled-in kernels, so registered bodies run in the same
